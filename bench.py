@@ -8,7 +8,7 @@ through [256, 512) (seq_len 512) after a 256-token prefill.  Workload = BASELINE
 slices, one rank per GPU, and the activation is handed from rank r to r+1 by one NCCL send/recv
 (configs[2] at N=4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # this framework
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]     # this framework
     python bench.py --impl reference [...]                          # the reference's CPU path
 
 Prints ONE JSON line (rank 0).  `value` = tokens/s with the activation resident in HBM;
@@ -84,6 +84,14 @@ def slice_file(shape_name: str, a: int, b: int) -> str:
 
 def synth_inputs(n: int, n_embd: int, seed: int) -> np.ndarray:
     return np.random.default_rng([SEED, seed]).standard_normal((n, n_embd), dtype=np.float32)
+
+
+def dump_outputs(d: str, **arrays) -> None:
+    """--dump-outputs: one DIR/<name>.npy per array, float32, so that two builds run with the same arguments (hence the
+    same seeded weights and inputs) can be compared output for output."""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a, np.float32))
 
 
 def measured_peak():
@@ -232,7 +240,9 @@ def run_reference(args):
         return 0
     sh = ggjt.SHAPES["7b"]
     path = slice_file("7b", 0, sh.n_layer - 1)
-    r = cpu_reference_run(path, sh.n_embd, args.steps, args.warmup)
+    r, _, _, outs = cpu_reference_run(path, sh.n_embd, args.steps, args.warmup, want_outputs=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, hidden_state=outs[-1])
     line = {"impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": r["steps"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
             "scaling": "strong", "vs_baseline": None, "dtype": "q4_0*q8_0->f32", "data": "synthetic",
@@ -342,6 +352,12 @@ def run_b200(args):
         dist.all_reduce(lt)
         launches = int(lt[0])
     value = K / (dev_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # what the last timed step returned to its caller: the model's hidden state for that token (the last slice's
+        # output, which the ring hands back to rank 0 at N > 1); read before the legs below reuse the buffers
+        last = np.empty((1, E), np.float32)
+        _d2h(sl, last)
+        dump_outputs(args.dump_outputs, hidden_state=last)
     pos_timed = [PREFILL + (i % cycle) for i in range(W, W + K)]
     timed_positions = ("%d..%d" % (pos_timed[0], pos_timed[-1]) if K <= cycle - (W % cycle) else
                        "%d..%d cyclically (%d steps)" % (PREFILL, N_CTX - 1, K))
@@ -663,6 +679,8 @@ def main():
     ap.add_argument("--warmup", type=int, default=8)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the hidden state the last one computed to DIR/hidden_state.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
