@@ -87,7 +87,8 @@ def lib() -> C.CDLL:
                            ("b200_extra_dims", [vp, C.POINTER(ci), C.POINTER(ci)]),
                            ("b200_extra_embed", [vp, vp, ci, vp]), ("b200_extra_logits", [vp, vp, ci, ci, vp]),
                            ("b200_extra_next_token", [vp, vp, ci, C.POINTER(C.c_int32)]),
-                           ("b200_extra_tokenize", [vp, C.c_char_p, vp, ci])):
+                           ("b200_extra_tokenize", [vp, C.c_char_p, vp, ci]),
+                           ("b200_debug_fast_matmul", [vp, ci, ci, ci, vp, ci, vp, vp, vp])):
             if hasattr(L, name):
                 getattr(L, name).argtypes = args
         if hasattr(L, "b200_extra_token_text"):
@@ -214,6 +215,22 @@ class Slice:
         out = np.zeros(count, np.uint32)
         check(lib().b200_debug_read(self._h, which, 0, count, _ptr(out)))
         return out.view(dtype)
+
+    def debug_fast_matmul(self, layer: int, which: int, x: np.ndarray, resid: Optional[np.ndarray] = None, tile: int = 0):
+        """One fast-mode weight matmul (which: 0 qkv, 1 wo, 2 w1|w3, 3 w2) -> (y, xh).  y is
+        [round_up(n_tokens, 256)][rows] float32, rows past n_tokens hold the sentinel 0xFFFFFFFF; xh is the fp16
+        activation operand [n_tokens][K]."""
+        i = self.info
+        K = i.n_ff if which == 3 else i.n_embd
+        rows = (3 * i.n_embd, i.n_embd, i.n_ff, i.n_embd)[which] if 0 <= which <= 3 else 0
+        x = np.ascontiguousarray(x, dtype=np.float32).reshape(-1, K)
+        n = x.shape[0]
+        r = None if resid is None else np.ascontiguousarray(resid, dtype=np.float32).reshape(n, i.n_embd)
+        y = np.empty(((n + 255) // 256 * 256, rows), np.float32)
+        xh = np.empty((n, K), np.float16)
+        check(lib().b200_debug_fast_matmul(self._h, layer, which, tile, _ptr(x), n, None if r is None else _ptr(r),
+                                           _ptr(y), _ptr(xh)))
+        return y, xh
 
     def skip_attention(self, on: bool) -> None:
         check(lib().b200_debug_skip_attention(self._h, int(on)))

@@ -414,19 +414,33 @@ static int launch_fast_gemm2_t(b200_slice * s, const PackedW & W, const float * 
     s->launches++;
     return 0;
 }
+// tile: 0 picks the token tile below; 128 / 256 force it (v2 only; b200_debug_fast_matmul)
 template <int EPI>
-static int launch_fast_any(b200_slice * s, const PackedW & W, const float * resid, int ldr, float * y, int ldy, int N, int out_rows) {
+static int launch_fast_any(b200_slice * s, const PackedW & W, const float * resid, int ldr, float * y, int ldy, int N, int out_rows,
+                           int tile = 0) {
     if (s->fast_version >= 2) {
         // 256-token tiles halve the dequantisation per flop; a matrix whose 128-row tiles x 256-token tiles would leave SMs idle
         // (wo, w2: 32 row tiles) takes 128-token tiles and three stages instead
         const int mtiles = (W.n_tiles * W.TR + 15) / 16;
-        const bool wide = (long long) mtiles * ((N + 255) / 256) >= s->n_sm || N <= 128;
+        const bool wide = tile ? tile == 256 : (long long) mtiles * ((N + 255) / 256) >= s->n_sm || N <= 128;
         if (W.wtype == kWT_Q4_0) return wide ? launch_fast_gemm2_t<kWT_Q4_0, EPI, 256>(s, W, resid, ldr, y, ldy, N, out_rows)
                                              : launch_fast_gemm2_t<kWT_Q4_0, EPI, 128>(s, W, resid, ldr, y, ldy, N, out_rows);
         return wide ? launch_fast_gemm2_t<kWT_Q8_0, EPI, 256>(s, W, resid, ldr, y, ldy, N, out_rows)
                     : launch_fast_gemm2_t<kWT_Q8_0, EPI, 128>(s, W, resid, ldr, y, ldy, N, out_rows);
     }
     return launch_fast_gemm<EPI>(s, W, resid, ldr, y, ldy, N, out_rows);
+}
+
+// The slice's weights suit the tcgen05 matmuls: Q4_0 (v1, v2) or Q8_0 (v2), and qkv / wo / w1|w3 are whole 16-group M tiles.
+static bool fast_weights_ok(const b200_slice * s, const LayerW & Lw) {
+    return (s->wtype == kWT_Q4_0 || (s->wtype == kWT_Q8_0 && s->fast_version >= 2)) && (Lw.qkv.n_tiles * Lw.qkv.TR) % 16 == 0 &&
+           (Lw.wo.n_tiles * Lw.wo.TR) % 16 == 0 && (Lw.w13.n_tiles * Lw.w13.TR) % 16 == 0;
+}
+
+// A call runs in fast mode only as a prompt chunk of one sequence: single-token steps and batched steps (one token for each of
+// several sessions, s->cols) promise results bit-identical to exact mode, so they never take it, whatever fast_min_tokens says.
+static bool fast_applicable(const b200_slice * s, const LayerW & Lw, int N) {
+    return s->fast_prefill && N > 1 && !s->cols && N >= s->fast_min_tokens && fast_weights_ok(s, Lw);
 }
 
 // ---------------------------------------------------------------- persistent single-token step (persist.cuh)
@@ -525,9 +539,7 @@ static int enqueue_layers(b200_slice * s, const float * in, int N, float * out) 
     for (int il = 0; il < (persist ? 0 : s->L); il++) {
         LayerW & Lw = s->layers[il];
         // grid-barrier norm+quant epilogue: decode only (every CTA of wo / w2 must be co-resident: 1 tile per CTA)
-        const bool fast = s->fast_prefill && N >= s->fast_min_tokens && (s->wtype == kWT_Q4_0 || (s->wtype == kWT_Q8_0 && s->fast_version >= 2)) &&
-                          (Lw.qkv.n_tiles * Lw.qkv.TR) % 16 == 0 &&
-                          (Lw.wo.n_tiles * Lw.wo.TR) % 16 == 0 && (Lw.w13.n_tiles * Lw.w13.TR) % 16 == 0;
+        const bool fast = fast_applicable(s, Lw, N);
         const bool nq = s->use_nq && N == 1 && !s->cols && s->wtype != kWT_F16 && Lw.wo.n_tiles <= 256 && Lw.wo.n_tiles <= s->n_sm * 2;
         float * nxt = (il == s->L - 1) ? out : ((il & 1) ? s->xb : s->xa);
         // cols mode (batched independent sequences): the kernels add session * sess_stride themselves
@@ -1490,6 +1502,62 @@ int b200_debug_read(b200_slice_t * s, int which, size_t offset_words, size_t cou
     B200_CUDA(cudaStreamSynchronize(s->stream));
     B200_CUDA(cudaMemcpy(out, (const uint32_t *) src[which] + offset_words, count * 4, cudaMemcpyDeviceToHost));
     return 0;
+}
+
+/* Test hook: ONE fast-mode weight matmul of `layer` with the launch sequence enqueue_layers uses (k_prep_q8_f16, then the
+ * tcgen05 kernel), on private buffers: the KV cache and n_past are not touched.  which: 0 qkv, 1 wo, 2 w1|w3, 3 w2. */
+int b200_debug_fast_matmul(b200_slice_t * s, int layer, int which, int tile, const float * x, int n_tokens, const float * resid,
+                           float * y, uint16_t * xh) {
+    if (!s || !x || !y || !xh) return fail(B200_EINVAL, "null argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    if (layer < 0 || layer >= s->L) return fail(B200_EINVAL, "layer %d outside [0, %d)", layer, s->L);
+    if (which < 0 || which > 3) return fail(B200_EINVAL, "bad matrix id %d", which);
+    if (n_tokens <= 0 || n_tokens > s->n_ctx) return fail(B200_EINVAL, "n_tokens %d outside [1, n_ctx %d]", n_tokens, s->n_ctx);
+    if (tile != 0 && tile != 128 && !(tile == 256 && s->fast_version >= 2))
+        return fail(B200_EINVAL, "token tile %d not available (fast kernel v%d)", tile, s->fast_version);
+    LayerW & Lw = s->layers[layer];
+    if (!fast_weights_ok(s, Lw)) return fail(B200_EINVAL, "this slice does not qualify for fast mode");
+    const bool has_resid = which == 1 || which == 3;
+    if (has_resid && !resid) return fail(B200_EINVAL, "wo / w2 need the residual input");
+    const int E = s->E, FF = s->FF, N = n_tokens;
+    const int K = which == 3 ? FF : E, rows = which == 0 ? 3 * E : (which == 2 ? FF : E);
+    const size_t n_pad = (size_t)(N + 255) & ~(size_t) 255;
+    B200_CUDA(cudaSetDevice(s->device));
+    float * d_x = nullptr, * d_r = nullptr, * d_y = nullptr;
+    auto run = [&]() -> int {
+        B200_CUDA(cudaMalloc(&d_x, (size_t) N * K * 4));
+        B200_CUDA(cudaMalloc(&d_y, n_pad * rows * 4));
+        if (has_resid) B200_CUDA(cudaMalloc(&d_r, (size_t) N * E * 4));
+        B200_CUDA(cudaMemcpyAsync(d_x, x, (size_t) N * K * 4, cudaMemcpyHostToDevice, s->stream));
+        if (has_resid) B200_CUDA(cudaMemcpyAsync(d_r, resid, (size_t) N * E * 4, cudaMemcpyHostToDevice, s->stream));
+        B200_CUDA(cudaMemsetAsync(d_y, 0xFF, n_pad * rows * 4, s->stream));      // sentinel: every word 0xFFFFFFFF (a NaN)
+        int rc;
+        switch (which) {
+        case 0:
+            if ((rc = launch_prep<true>(s, d_x, E, Lw.attn_norm, E, N))) return rc;
+            if ((rc = launch_fast_any<FG_STORE>(s, Lw.qkv, nullptr, 0, d_y, 3 * E, N, 3 * E, tile))) return rc;
+            break;
+        case 1:
+            if ((rc = launch_prep<false>(s, d_x, E, nullptr, E, N))) return rc;
+            if ((rc = launch_fast_any<FG_RESID>(s, Lw.wo, d_r, E, d_y, E, N, E, tile))) return rc;
+            break;
+        case 2:
+            if ((rc = launch_prep<true>(s, d_x, E, Lw.ffn_norm, E, N))) return rc;
+            if ((rc = launch_fast_any<FG_GATE>(s, Lw.w13, nullptr, 0, d_y, FF, N, FF, tile))) return rc;
+            break;
+        default:
+            if ((rc = launch_prep<false>(s, d_x, FF, nullptr, FF, N))) return rc;
+            if ((rc = launch_fast_any<FG_RESID>(s, Lw.w2, d_r, E, d_y, E, N, E, tile))) return rc;
+        }
+        B200_CUDA(cudaMemcpyAsync(y, d_y, n_pad * rows * 4, cudaMemcpyDeviceToHost, s->stream));
+        B200_CUDA(cudaMemcpyAsync(xh, s->xh, (size_t) N * K * 2, cudaMemcpyDeviceToHost, s->stream));
+        B200_CUDA(cudaStreamSynchronize(s->stream));
+        return 0;
+    };
+    const int rc = run();
+    if (rc) cudaStreamSynchronize(s->stream);
+    cudaFree(d_x); cudaFree(d_y); cudaFree(d_r);
+    return rc;
 }
 
 }  // extern "C"

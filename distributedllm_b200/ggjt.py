@@ -354,6 +354,7 @@ SHAPES = {
     "tiny3b": ModelShape(512, 800, 32, 8, 3),        # d_head 100 (OpenLLaMA-3B-like head), n_ff 2144 = 67 blocks
     "tiny128": ModelShape(512, 512, 32, 4, 3),       # d_head 128 (the 7B/13B head size), n_ff 1376 = 43 blocks
     "tiny128b": ModelShape(512, 512, 64, 4, 2),      # d_head 128, n_ff 1408: every matrix is a whole number of 128-row MMA tiles
+    "tiny128c": ModelShape(512, 512, 320, 4, 2),     # d_head 128, n_ff 1600 = 12.5 x 128: w2's last 128-wide K block is half empty
     "3b":     ModelShape(32000, 3200, 216, 32, 26),  # OpenLLaMA-3B: n_ff 8640
     "7b":     ModelShape(32000, 4096, 256, 32, 32),
     "13b":    ModelShape(32000, 5120, 256, 40, 40),

@@ -103,8 +103,11 @@ int b200_batch_forward_device(b200_slice_t * s, const int * sessions, int n_seq,
 
 /* Fast mode for prefill calls (n_tokens >= min_tokens): the Q4_0 / Q8_0 weight matmuls run on the tcgen05 tensor cores with
  * the dequantisation fused in (csrc/fastgemm2.cuh; Q4_1 and F16 slices ignore the switch and stay exact).  NOT bit-exact: operands are rounded to fp16 after the reference's
- * Q8_0 activation quantisation; deviation from exact mode is bounded in tests/test_gpu_fast_prefill.py.  Off by default
- * (or B200_FAST_PREFILL=1); decode steps always run in exact mode. */
+ * Q8_0 activation quantisation; deviation from exact mode is bounded in tests/test_gpu_fast_prefill.py and, one matmul at a
+ * time, in tests/test_gpu_fast_matmul.py.  The fp16 operands limit the un-normalised inputs of wo and w2 to |x| <= 65504;
+ * beyond that fast mode overflows where exact mode stays finite.  Off by default (or B200_FAST_PREFILL=1).  Single-token
+ * steps and batched steps (b200_batch_forward*) always run in exact mode, whatever min_tokens is: only a multi-token call of
+ * one sequence takes the fast path. */
 int b200_slice_set_fast_prefill(b200_slice_t * s, int on, int min_tokens);
 
 /* Block until everything queued on the slice's stream has finished. */
@@ -136,6 +139,17 @@ float * b200_slice_dev_out(b200_slice_t * s);
 /* Test hook: copy `count` 32-bit words of an internal activation buffer to the host after a forward
  * (0 qkv, 1 att, 2 ffin, 3 gate, 4 xa, 5 xb, 6 q16, 7 k-cache, 8 v-cache).  Not part of the drop-in surface. */
 int b200_debug_read(b200_slice_t * s, int which, size_t offset_words, size_t count, void * out);
+
+/* Test hook: run ONE fast-mode weight matmul of `layer` (0-based within the slice) on private buffers, with the launch
+ * sequence a fast prefill uses; the KV cache and n_past are untouched.  which: 0 qkv (RMSNorm by attention_norm, x is
+ * [n_tokens][n_embd], y has 3 n_embd rows), 1 wo (x [n_tokens][n_embd], y = W x + resid), 2 w1|w3 (RMSNorm by ffn_norm,
+ * y = silu(w1 x) * (w3 x), n_ff rows), 3 w2 (x [n_tokens][n_ff], y = W x + resid).  resid is [n_tokens][n_embd] (wo, w2 only).
+ * tile: 0 = the token tile a forward would pick, 128 / 256 force one (256 needs the default v2 kernel).
+ * y receives [round_up(n_tokens, 256)][rows] floats; rows past n_tokens keep the sentinel 0xFFFFFFFF (a NaN).
+ * xh receives the fp16 activation operand [n_tokens][K] (K = n_ff for w2, else n_embd).
+ * B200_EINVAL when the slice's weights do not qualify for fast mode. */
+int b200_debug_fast_matmul(b200_slice_t * s, int layer, int which, int tile, const float * x, int n_tokens, const float * resid,
+                           float * y, uint16_t * xh);
 
 /* Measurement aid (bench.py roofline): while on, a decode step launches only its weight-matmul kernels. */
 int b200_debug_skip_attention(b200_slice_t * s, int on);

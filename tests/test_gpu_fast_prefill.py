@@ -64,6 +64,71 @@ def test_tensor_core_matmul_alone_is_tight(tmp_models, monkeypatch, version, wty
     b.close()
 
 
+def _bits(a):
+    return np.ascontiguousarray(a, dtype=np.float32).view(np.uint32)
+
+
+@pytest.mark.parametrize("via_env", [False, True], ids=["set_fast_prefill", "B200_FAST_MIN_TOKENS"])
+def test_single_token_steps_stay_exact_at_min_tokens_one(tmp_models, monkeypatch, via_env):
+    """Decode steps never take the tensor-core path, even when fast mode would accept one-token calls."""
+    from distributedllm_b200 import capi
+    sh = ggjt.SHAPES["tiny128b"]
+    path = tmp_models("tiny128b", ggjt.T_Q4_0, 0, 1)
+    rng = np.random.default_rng(6)
+    prompt = rng.standard_normal((20, sh.n_embd), dtype=np.float32)
+    exact = capi.Slice(path, 0, 128)
+    if via_env:
+        monkeypatch.setenv("B200_FAST_MIN_TOKENS", "1")
+    fast = capi.Slice(path, 0, 128)
+    assert (_bits(exact.forward(prompt)) == _bits(fast.forward(prompt))).all()      # fast mode still off: same cache
+    if via_env:
+        fast.set_fast_prefill(True)
+    else:
+        fast.set_fast_prefill(True, 1)
+    for step in range(6):                                  # the first step captures the decode graph with fast mode on
+        t = rng.standard_normal((1, sh.n_embd), dtype=np.float32)
+        assert (_bits(exact.forward(t)) == _bits(fast.forward(t))).all(), step
+    exact.close()
+    fast.close()
+
+
+def test_fast_path_starts_exactly_at_min_tokens(tmp_models):
+    """A call of min_tokens - 1 tokens is exact mode bit for bit; a call of min_tokens tokens runs fast."""
+    from distributedllm_b200 import capi
+    sh = ggjt.SHAPES["tiny128b"]
+    path = tmp_models("tiny128b", ggjt.T_Q4_0, 0, 1)
+    x = np.random.default_rng(7).standard_normal((40, sh.n_embd), dtype=np.float32)
+    for n, same in ((39, True), (40, False)):
+        exact, fast = capi.Slice(path, 0, 128), capi.Slice(path, 0, 128)
+        fast.set_fast_prefill(True, 40)
+        ye, yf = exact.forward(x[:n]), fast.forward(x[:n])
+        assert bool((_bits(ye) == _bits(yf)).all()) == same, n
+        exact.close()
+        fast.close()
+
+
+@pytest.mark.parametrize("version,wtype", [(2, ggjt.T_Q4_0), (2, ggjt.T_Q8_0), (1, ggjt.T_Q4_0)],
+                         ids=["v2-q4_0", "v2-q8_0", "v1-q4_0"])
+def test_fast_prefill_is_deterministic(tmp_models, monkeypatch, version, wtype):
+    """Two handles fed the same prompt agree bit for bit, and so do session 2 of one handle and session 0 of another."""
+    from distributedllm_b200 import capi
+    monkeypatch.setenv("B200_FAST_V", str(version))
+    sh = ggjt.SHAPES["tiny128b"]
+    path = tmp_models("tiny128b", wtype, 0, 1)
+    rng = np.random.default_rng(8)
+    chunks = [rng.standard_normal((n, sh.n_embd), dtype=np.float32) for n in (300, 100)]
+    a, b = capi.Slice(path, 0, 512, n_sessions=3), capi.Slice(path, 0, 512)
+    c = capi.Slice(path, 0, 512)
+    for s in (a, b, c):
+        s.set_fast_prefill(True, 32)
+    for x in chunks:
+        yb = b.forward(x)
+        assert (_bits(yb) == _bits(c.forward(x))).all()
+        assert (_bits(yb) == _bits(a.session_forward(2, x))).all()
+    for s in (a, b, c):
+        s.close()
+
+
 def test_fast_mode_falls_back_when_shapes_do_not_tile(tmp_models):
     """tiny128 has n_ff = 1376 (not a multiple of 64): the request is honoured with the exact kernels."""
     from distributedllm_b200 import capi

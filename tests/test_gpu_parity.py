@@ -47,6 +47,20 @@ def test_bit_exact_prefill_then_decode(tmp_models, shape, wtype):
     assert bad == 0, "%d of %d floats differ from the oracle" % (bad, tot)
 
 
+@pytest.mark.parametrize("wtype,version", [(ggjt.T_Q4_1, 2), (ggjt.T_F16, 2), (ggjt.T_Q8_0, 1)],
+                         ids=["q4_1", "f16", "q8_0-v1"])
+def test_fast_prefill_switch_keeps_other_types_exact(tmp_models, monkeypatch, wtype, version):
+    """Fast mode covers Q4_0 (and Q8_0 with the v2 kernel) only; every other slice ignores the switch and stays
+    bit-identical to the oracle.  tiny128b passes the shape test, so only the weight type decides."""
+    monkeypatch.setenv("B200_FAST_PREFILL", "1")
+    monkeypatch.setenv("B200_FAST_MIN_TOKENS", "2")
+    monkeypatch.setenv("B200_FAST_V", str(version))
+    sh = ggjt.SHAPES["tiny128b"]
+    path = tmp_models("tiny128b", wtype, 0, 1)
+    bad, tot = _run_pair(path, [40, 1, 1, 7, 1, 130, 3, 1], sh)
+    assert bad == 0, "%d of %d floats differ from the oracle" % (bad, tot)
+
+
 def test_ring_and_simple_kernels_agree(tmp_models, monkeypatch):
     sh = ggjt.SHAPES["tiny3b"]
     path = tmp_models("tiny3b", ggjt.T_Q4_0, 0, 2)

@@ -49,6 +49,27 @@ def test_batched_step_equals_private_contexts(tmp_models, shape, wtype):
     gpu.close()
 
 
+def test_batched_step_stays_exact_with_fast_prefill_on(tmp_models):
+    """A batched step of 40 sessions has more columns than fast mode's min_tokens (32), yet it is 40 single-token steps:
+    with fast prefill on it stays bit-identical to the same batch with fast prefill off."""
+    from distributedllm_b200 import capi
+    sh = ggjt.SHAPES["tiny128b"]
+    path = tmp_models("tiny128b", ggjt.T_Q4_0, 0, 1, seed=23)
+    B = 40
+    fast, exact = capi.Slice(path, 0, 64, n_sessions=B), capi.Slice(path, 0, 64, n_sessions=B)
+    rng = np.random.default_rng(5)
+    for k in range(B):                                   # prompts shorter than min_tokens: exact on both handles
+        x = rng.standard_normal((1 + k % 7, sh.n_embd), dtype=np.float32)
+        assert (_bits(fast.session_forward(k, x)) == _bits(exact.session_forward(k, x))).all()
+    fast.set_fast_prefill(True, 32)
+    sessions = list(rng.permutation(B))
+    for step in range(3):
+        x = rng.standard_normal((B, sh.n_embd), dtype=np.float32)
+        assert (_bits(fast.batch_forward(sessions, x)) == _bits(exact.batch_forward(sessions, x))).all(), step
+    fast.close()
+    exact.close()
+
+
 def test_session_zero_is_the_reference_context_and_errors(tmp_models):
     from distributedllm_b200 import capi
     sh = ggjt.SHAPES["tiny128"]
