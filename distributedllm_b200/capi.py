@@ -49,6 +49,8 @@ def lib() -> C.CDLL:
         L.b200_session_forward_device.argtypes = [vp, ci, vp, ci, vp, ci]
         L.b200_batch_forward.argtypes = [vp, vp, ci, vp, vp]
         L.b200_batch_forward_device.argtypes = [vp, vp, ci, vp, vp, ci]
+        L.b200_mixed_forward.argtypes = [vp, vp, vp, ci, vp, vp]
+        L.b200_mixed_forward_device.argtypes = [vp, vp, vp, ci, vp, vp, ci]
         L.b200_slice_unload.argtypes = [vp]
         L.b200_slice_clear.argtypes = [vp]
         L.b200_slice_rewind.argtypes = [vp, ci]
@@ -82,7 +84,8 @@ def lib() -> C.CDLL:
                            ("b200_pipeline_step", [vp, vp, ci, ci]),
                            ("b200_pipeline_mailbox_export", [vp, vp]), ("b200_pipeline_mailbox_connect", [vp, vp, ci]),
                            ("b200_pipeline_collect", [vp, ci, vp]), ("b200_pipeline_pingpong", [vp, ci, ci, vp]), ("b200_pipeline_transport", [vp]), ("b200_pipeline_set_transport", [vp, ci]), ("b200_pipeline_error", [vp]),
-                           ("b200_pipeline_step_session", [vp, ci, vp, ci, ci]), ("b200_pipeline_step_batch", [vp, vp, ci, vp, ci]), ("b200_pipeline_destroy", [vp]),
+                           ("b200_pipeline_step_session", [vp, ci, vp, ci, ci]), ("b200_pipeline_step_batch", [vp, vp, ci, vp, ci]),
+                           ("b200_pipeline_step_mixed", [vp, vp, vp, ci, vp, ci]), ("b200_pipeline_destroy", [vp]),
                            ("b200_extra_load", [C.c_char_p, ci, C.POINTER(vp)]), ("b200_extra_unload", [vp]),
                            ("b200_extra_dims", [vp, C.POINTER(ci), C.POINTER(ci)]),
                            ("b200_extra_embed", [vp, vp, ci, vp]), ("b200_extra_logits", [vp, vp, ci, ci, vp]),
@@ -105,6 +108,14 @@ def check(rc: int) -> None:
 
 def _ptr(a: np.ndarray) -> C.c_void_p:
     return C.c_void_p(a.ctypes.data)
+
+
+def _segments(sessions, n_tokens):
+    ids = np.ascontiguousarray(sessions, dtype=np.int32).reshape(-1)
+    lens = np.ascontiguousarray(n_tokens, dtype=np.int32).reshape(-1)
+    if ids.shape != lens.shape:
+        raise ValueError("mixed step: %d sessions but %d token counts" % (ids.size, lens.size))
+    return ids, lens
 
 
 class Slice:
@@ -134,6 +145,18 @@ class Slice:
     def batch_forward_device(self, sessions, d_in: int, d_out: int, sync: bool = False) -> None:
         ids = np.ascontiguousarray(sessions, dtype=np.int32)
         check(lib().b200_batch_forward_device(self._h, _ptr(ids), len(ids), C.c_void_p(d_in), C.c_void_p(d_out), int(sync)))
+
+    def mixed_forward(self, sessions, n_tokens, x: np.ndarray) -> np.ndarray:
+        """n_tokens[i] tokens of sessions[i] in one pass: x is [sum(n_tokens)][n_embd], the segments back to back."""
+        ids, lens = _segments(sessions, n_tokens)
+        x = np.ascontiguousarray(x, dtype=np.float32).reshape(int(lens.sum()), self.n_embd)
+        out = np.empty_like(x)
+        check(lib().b200_mixed_forward(self._h, _ptr(ids), _ptr(lens), len(ids), _ptr(x), _ptr(out)))
+        return out
+
+    def mixed_forward_device(self, sessions, n_tokens, d_in: int, d_out: int, sync: bool = False) -> None:
+        ids, lens = _segments(sessions, n_tokens)
+        check(lib().b200_mixed_forward_device(self._h, _ptr(ids), _ptr(lens), len(ids), C.c_void_p(d_in), C.c_void_p(d_out), int(sync)))
 
     def session_n_past(self, session: int) -> int:
         return lib().b200_session_n_past(self._h, session)

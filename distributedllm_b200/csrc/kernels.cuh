@@ -1263,7 +1263,7 @@ struct RopeArgs {
     const int * n_past;
     const float2 * cs;            // [n_ctx][D/2] (cos, sin)
     uint16_t * q16; uint16_t * kc; uint16_t * vc;   // kc/vc: this layer's cache base
-    const int2 * cols; size_t sess_stride;          // batched step: column n = (session, position); cache base += session * stride
+    const int4 * cols; size_t sess_stride;          // multi-session step: column n = (session, position, T, 0); cache base += session * stride
 };
 
 __global__ void k_rope_append(const RopeArgs a) {
@@ -1271,7 +1271,7 @@ __global__ void k_rope_append(const RopeArgs a) {
     grid_dep_wait();
     const int n = blockIdx.y, half = a.D / 2;
     int pos; uint16_t * kcb = a.kc, * vcb = a.vc;
-    if (a.cols) { const int2 c = a.cols[n]; pos = c.y; kcb += (size_t) c.x * a.sess_stride; vcb += (size_t) c.x * a.sess_stride; }
+    if (a.cols) { const int4 c = a.cols[n]; pos = c.y; kcb += (size_t) c.x * a.sess_stride; vcb += (size_t) c.x * a.sess_stride; }
     else pos = *a.n_past + n;
     const float * row = a.qkv + (size_t) n * 3 * a.E;
     for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < a.E / 2; p += gridDim.x * blockDim.x) {
@@ -1302,7 +1302,7 @@ struct AttnArgs {
     const uint16_t * texp;
     float * out;                  // [N][E]
     float kq_scale;
-    const int2 * cols; size_t sess_stride;   // batched step (independent sequences): column n = (session, position), T = position + 1
+    const int4 * cols; size_t sess_stride;   // multi-session step: column n = (session, position, T, 0), tcount = position + 1
 };
 
 __global__ void __launch_bounds__(512) k_attention(const AttnArgs a) {
@@ -1311,7 +1311,7 @@ __global__ void __launch_bounds__(512) k_attention(const AttnArgs a) {
     grid_dep_wait();
     const int h = blockIdx.x, n = blockIdx.y, D = a.D, E = a.E;
     int T, tcount; const uint16_t * kcb = a.kc, * vcb = a.vc;
-    if (a.cols) { const int2 c = a.cols[n]; T = tcount = c.y + 1; kcb += (size_t) c.x * a.sess_stride; vcb += (size_t) c.x * a.sess_stride; }
+    if (a.cols) { const int4 c = a.cols[n]; T = c.z; tcount = c.y + 1; kcb += (size_t) c.x * a.sess_stride; vcb += (size_t) c.x * a.sess_stride; }
     else { const int n_past = *a.n_past; T = n_past + a.N; tcount = n_past + n + 1; }
     float * sc = (float *) smem;                                   // [T]
     uint16_t * p16 = (uint16_t *)(sc + ((T + 3) & ~3));            // [T]
@@ -1425,7 +1425,9 @@ struct Attn128Args {
     int out_soff;                                                    // Q4_1 weights: Q8_1 instead, block sums at da_out + out_soff
     int n_ctx; float kq_scale;
     unsigned long long * trace;
-    const int2 * cols; size_t sess_stride;   // batched step (FUSE only): column n = (session, position); each column is an N = 1 step
+    // multi-session step: column n = (session, position, T, 0).  FUSE: every column is an N = 1 step (T = position + 1);
+    // !FUSE: launch column ny is colmap[n0 + ny], the columns of a mixed step that are not on the tiled kernel
+    const int4 * cols; size_t sess_stride; const int * colmap;
     int pf_rows;                  // FUSE: rows of this CTA's K / V share staged in shared memory ahead of the dependency wait
     int lut_smem;                 // FUSE: also stage the negative half of the exp table (64 KB) -- softmax arguments are <= 0
 };
@@ -1472,10 +1474,10 @@ __global__ void __cluster_dims__(4, 1, 1) __launch_bounds__(256) k_attn128(const
     // after their own dependency wait (see k_gemv).  So when this code runs, every kernel up to the one before qkv has
     // finished: the position counter is final and all cache rows < pos are final.  Only the qkv row itself needs the wait.
     if (!FUSE) grid_dep_wait();
-    const int h = blockIdx.x >> 2, g = blockIdx.x & 3, ny = blockIdx.y, n = a.n0 + ny, E = a.E;
+    const int h = blockIdx.x >> 2, g = blockIdx.x & 3, ny = blockIdx.y, n = a.colmap ? a.colmap[a.n0 + ny] : a.n0 + ny, E = a.E;
     int T, tcount, pos;
     uint16_t * kc = a.kc, * vc = a.vc;
-    if (a.cols) { const int2 c = a.cols[n]; pos = c.y; T = tcount = pos + 1; kc += (size_t) c.x * a.sess_stride; vc += (size_t) c.x * a.sess_stride; }
+    if (a.cols) { const int4 c = a.cols[n]; pos = c.y; T = c.z; tcount = pos + 1; kc += (size_t) c.x * a.sess_stride; vc += (size_t) c.x * a.sess_stride; }
     else { const int n_past = *a.n_past; T = n_past + a.N; tcount = n_past + n + 1; pos = n_past + n; }
     float * sc = (float *) smem;                                   // [T]
     uint16_t * p16 = (uint16_t *)(sc + ((T + 3) & ~3));            // [T]
@@ -1761,9 +1763,14 @@ __global__ void __launch_bounds__(1024) k_peer_send(const PeerSendArgs a) {
 //   V.p      32 f32 slots per channel (slot = t mod 32, vector j = slot / 8 -> warp-quad g), positions in ascending order,
 //            ((p0+p2)+(p1+p3)) per slot, the 8-slot tree, the (T mod 32) tail in double -- T = n_past + N of the CALL
 // Needs T = n_past + N <= kAttnTMax staged rows (139 KB); longer contexts keep the per-query cluster kernel.
+// A mixed step (prompt chunks of several sessions in one pass) hands the kernel a table of query blocks: block y holds nq
+// consecutive columns of ONE segment, and carries that segment's session (whose cache the CTA stages) and T.  A prompt chunk
+// of one sequence is the one-segment case: no table, blocks of kAttnQB columns at the device-side position *n_past.
 // =============================================================================================
 constexpr int kAttnQB = 16;
 constexpr int kAttnTMax = 512;
+
+struct AttnBlock { int col0, nq, session, pos0, T; };   // first column, queries, session, position of the first query, T
 
 struct AttnTiledArgs {
     const uint16_t * q16; const uint16_t * kc; const uint16_t * vc;
@@ -1772,18 +1779,27 @@ struct AttnTiledArgs {
     float * out;                                   // [N][E]
     int * aq_out; float * da_out; int out_nbq; float out_dscale; int out_soff;
     float kq_scale;
-    int t_rows, t_pad;                             // staged rows (>= n_past + N) and the padded score row length
+    int t_rows, t_pad;                             // staged rows (>= the largest T) and the padded score row length
+    const AttnBlock * blocks; size_t sess_stride;  // mixed step: block table (grid.y entries); cache base += session * stride
 };
 
 __global__ void __launch_bounds__(512) k_attn128_tiled(const AttnTiledArgs a) {
     extern __shared__ __align__(16) uint8_t smem[];
     if (threadIdx.x == 0) grid_dep_launch();
     grid_dep_wait();
-    const int h = blockIdx.x, n0 = blockIdx.y * kAttnQB, E = a.E;
+    const int h = blockIdx.x, E = a.E;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int n_past = *a.n_past, T = n_past + a.N;
-    const int nq = min(kAttnQB, a.N - n0);                               // queries of this block
-    const int tmax = n_past + n0 + nq;                                   // positions the block's last query sees
+    int col0, nq, pos0, T;                                               // first column, queries, first query's position, T
+    const uint16_t * kc = a.kc, * vc = a.vc;
+    if (a.blocks) {
+        const AttnBlock b = a.blocks[blockIdx.y];
+        col0 = b.col0; nq = b.nq; pos0 = b.pos0; T = b.T;
+        kc += (size_t) b.session * a.sess_stride; vc += (size_t) b.session * a.sess_stride;
+    } else {
+        const int n_past = *a.n_past;
+        col0 = blockIdx.y * kAttnQB; nq = min(kAttnQB, a.N - col0); pos0 = n_past + col0; T = n_past + a.N;
+    }
+    const int tmax = pos0 + nq;                                          // positions the block's last query sees
     uint8_t * KV = smem;                                                 // [t_rows][kAttnRow]
     float * sc = (float *)(smem + (size_t) a.t_rows * kAttnRow);         // [QB][t_pad]
     uint16_t * p16 = (uint16_t *)(sc + (size_t) kAttnQB * a.t_pad);      // [QB][t_pad]
@@ -1793,11 +1809,11 @@ __global__ void __launch_bounds__(512) k_attn128_tiled(const AttnTiledArgs a) {
     // ---- stage the head's key rows t < tmax and the block's query rows
     for (int idx = tid; idx < tmax * 16; idx += 512) {
         const int t = idx >> 4, ch = idx & 15;
-        cp_async16(KV + (size_t) t * kAttnRow + ch * 16, a.kc + (size_t) t * E + h * 128 + ch * 8);
+        cp_async16(KV + (size_t) t * kAttnRow + ch * 16, kc + (size_t) t * E + h * 128 + ch * 8);
     }
     for (int idx = tid; idx < nq * 16; idx += 512) {
         const int q = idx >> 4, ch = idx & 15;
-        cp_async16(q16s + q * 128 + ch * 8, a.q16 + (size_t)(n0 + q) * E + h * 128 + ch * 8);
+        cp_async16(q16s + q * 128 + ch * 8, a.q16 + (size_t)(col0 + q) * E + h * 128 + ch * 8);
     }
     cp_async_wait_all();
     __syncthreads();
@@ -1806,7 +1822,7 @@ __global__ void __launch_bounds__(512) k_attn128_tiled(const AttnTiledArgs a) {
     {
         const int ql = tid & 3;
         for (int q = 0; q < nq; q++) {
-            const int tcount = n_past + n0 + q + 1;
+            const int tcount = pos0 + q + 1;
             float qf[4][8];
             #pragma unroll
             for (int c = 0; c < 4; c++)
@@ -1848,11 +1864,11 @@ __global__ void __launch_bounds__(512) k_attn128_tiled(const AttnTiledArgs a) {
     // ---- softmax: warp q owns query q; meanwhile the value rows replace the key rows
     for (int idx = tid; idx < tmax * 16; idx += 512) {
         const int t = idx >> 4, ch = idx & 15;
-        cp_async16(KV + (size_t) t * kAttnRow + ch * 16, a.vc + (size_t) t * E + h * 128 + ch * 8);
+        cp_async16(KV + (size_t) t * kAttnRow + ch * 16, vc + (size_t) t * E + h * 128 + ch * 8);
     }
     asm volatile("cp.async.commit_group;" ::: "memory");
     if (warp < nq) {
-        const int q = warp, tcount = n_past + n0 + q + 1;
+        const int q = warp, tcount = pos0 + q + 1;
         float * s_q = sc + (size_t) q * a.t_pad;
         uint16_t * p_q = p16 + (size_t) q * a.t_pad;
         float mx = -INFINITY;
@@ -1879,7 +1895,7 @@ __global__ void __launch_bounds__(512) k_attn128_tiled(const AttnTiledArgs a) {
     for (int q0 = 0; q0 < nq; q0 += 4) {
         const int q = q0 + grp;
         const bool live = q < nq;
-        const int n = n0 + q, tcount = n_past + n + 1, lim = live ? min(npT, tcount) : 0;
+        const int n = col0 + q, tcount = pos0 + q + 1, lim = live ? min(npT, tcount) : 0;
         const uint16_t * p_q = p16 + (size_t) q * a.t_pad;
         float acc[4][8];
         #pragma unroll
@@ -1935,8 +1951,13 @@ __global__ void k_advance_sent(int * n_past, int by, MailboxHdr * mine) {
     grid_dep_wait();
     if (threadIdx.x == 0) { *n_past += by; mine->seq_out = mine->seq_out + 1; }
 }
-// batched step: every listed session moves one position
-__global__ void k_advance_cols(int * n_past, const int2 * cols, int n) { grid_dep_wait(); if ((int) threadIdx.x < n) n_past[cols[threadIdx.x].x] += 1; }
+// multi-session step: the columns of one session are consecutive, so the last column of each segment sets that session's
+// counter to its position + 1 (= n_past + segment length); one writer per session
+__global__ void k_advance_segs(int * n_past, const int4 * cols, int n) {
+    grid_dep_wait();
+    for (int i = threadIdx.x; i < n; i += blockDim.x)
+        if (i == n - 1 || cols[i + 1].x != cols[i].x) n_past[cols[i].x] = cols[i].y + 1;
+}
 
 }  // namespace b200
 

@@ -203,6 +203,8 @@ static PyObject * py_propagate_forward_buffer(PyObject *, PyObject * args) {
 // ---- additive: several sequences on one node (n_sessions contexts over the same weights) ------------------
 // propagate_forward_session(session, float32 bytes-like) -> bytes        tokens of ONE session
 // propagate_forward_batch([sessions], float32 bytes-like) -> bytes       one token for EACH listed session, one pass
+// propagate_forward_mixed([sessions], [n_tokens], float32 bytes-like) -> bytes
+//                                                 n_tokens[i] tokens of sessions[i], segments back to back, one pass
 // clear_session(session)  (-1 = all)
 static PyObject * py_propagate_forward_session(PyObject *, PyObject * args) {
     int session; PyObject * values;
@@ -225,18 +227,24 @@ static PyObject * py_propagate_forward_session(PyObject *, PyObject * args) {
     return PyBytes_FromStringAndSize((const char *) y.data(), (Py_ssize_t)(y.size() * sizeof(float)));
 }
 
+static bool list_to_ints(PyObject * list, const char * what, std::vector<int> & out) {
+    if (!PyList_Check(list)) { PyErr_Format(PyExc_TypeError, "%s must be a list of int", what); return false; }
+    out.resize((size_t) PyList_Size(list));
+    for (size_t i = 0; i < out.size(); i++) {
+        const long v = PyLong_AsLong(PyList_GetItem(list, (Py_ssize_t) i));
+        if (v == -1 && PyErr_Occurred()) return false;
+        out[i] = (int) v;
+    }
+    return true;
+}
+
 static PyObject * py_propagate_forward_batch(PyObject *, PyObject * args) {
     PyObject * sessions, * values;
     if (!PyArg_ParseTuple(args, "OO", &sessions, &values)) return nullptr;
     SlicePtr sp = current_slice();
     if (!sp) { PyErr_SetString(PyExc_RuntimeError, "propagate_forward_batch: no slice loaded"); return nullptr; }
-    if (!PyList_Check(sessions)) { PyErr_SetString(PyExc_TypeError, "propagate_forward_batch: sessions must be a list of int"); return nullptr; }
-    std::vector<int> ids((size_t) PyList_Size(sessions));
-    for (size_t i = 0; i < ids.size(); i++) {
-        const long v = PyLong_AsLong(PyList_GetItem(sessions, (Py_ssize_t) i));
-        if (v == -1 && PyErr_Occurred()) return nullptr;
-        ids[i] = (int) v;
-    }
+    std::vector<int> ids;
+    if (!list_to_ints(sessions, "propagate_forward_batch: sessions", ids)) return nullptr;
     std::vector<float> x, y;
     if (!list_to_floats(values, x)) return nullptr;
     b200_slice_info_t info;
@@ -253,6 +261,39 @@ static PyObject * py_propagate_forward_batch(PyObject *, PyObject * args) {
     sp.reset();
     Py_END_ALLOW_THREADS
     if (rc) { PyErr_Format(PyExc_RuntimeError, "propagate_forward_batch: %s", err.c_str()); return nullptr; }
+    return PyBytes_FromStringAndSize((const char *) y.data(), (Py_ssize_t)(y.size() * sizeof(float)));
+}
+
+static PyObject * py_propagate_forward_mixed(PyObject *, PyObject * args) {
+    PyObject * sessions, * counts, * values;
+    if (!PyArg_ParseTuple(args, "OOO", &sessions, &counts, &values)) return nullptr;
+    SlicePtr sp = current_slice();
+    if (!sp) { PyErr_SetString(PyExc_RuntimeError, "propagate_forward_mixed: no slice loaded"); return nullptr; }
+    std::vector<int> ids, lens;
+    if (!list_to_ints(sessions, "propagate_forward_mixed: sessions", ids) || !list_to_ints(counts, "propagate_forward_mixed: n_tokens", lens))
+        return nullptr;
+    if (ids.size() != lens.size()) {
+        PyErr_SetString(PyExc_ValueError, "propagate_forward_mixed: need one token count per listed session");
+        return nullptr;
+    }
+    std::vector<float> x, y;
+    if (!list_to_floats(values, x)) return nullptr;
+    b200_slice_info_t info;
+    if (b200_slice_info(sp->h, &info)) return raise_b200("propagate_forward_mixed");
+    long long rows = 0;
+    for (int n : lens) rows += n;
+    if (rows < 0 || x.size() != (size_t) rows * info.n_embd) {
+        PyErr_SetString(PyExc_ValueError, "propagate_forward_mixed: need exactly sum(n_tokens) rows of n_embd floats");
+        return nullptr;
+    }
+    y.resize(x.size());
+    int rc; std::string err;
+    Py_BEGIN_ALLOW_THREADS
+    rc = b200_mixed_forward(sp->h, ids.data(), lens.data(), (int) ids.size(), x.data(), y.data());
+    if (rc) err = b200_last_error();
+    sp.reset();
+    Py_END_ALLOW_THREADS
+    if (rc) { PyErr_Format(PyExc_RuntimeError, "propagate_forward_mixed: %s", err.c_str()); return nullptr; }
     return PyBytes_FromStringAndSize((const char *) y.data(), (Py_ssize_t)(y.size() * sizeof(float)));
 }
 
@@ -364,6 +405,8 @@ static PyMethodDef Methods[] = {
     {"propagate_forward_buffer", py_propagate_forward_buffer, METH_VARARGS, "Same, float32 bytes-like in, bytes out"},
     {"propagate_forward_session", py_propagate_forward_session, METH_VARARGS, "(session, float32 buffer) -> bytes: tokens of one of B200_SESSIONS contexts"},
     {"propagate_forward_batch", py_propagate_forward_batch, METH_VARARGS, "([sessions], float32 buffer) -> bytes: one token for each listed session in one pass"},
+    {"propagate_forward_mixed", py_propagate_forward_mixed, METH_VARARGS,
+     "([sessions], [n_tokens], float32 buffer) -> bytes: n_tokens[i] tokens of sessions[i], segments back to back, in one pass"},
     {"clear_session", py_clear_session, METH_VARARGS, "Clear one session's context (-1: all)"},
     {"get_logits", py_get_logits, METH_VARARGS, "Apply the output layers to embeddings to get logits"},
     {"get_next_token", py_get_next_token, METH_VARARGS, "Greedy next token"},

@@ -38,6 +38,17 @@ struct LayerW {
 struct GraphKey { const float * in; float * out; int host; bool operator<(const GraphKey & o) const {
     return in != o.in ? in < o.in : (out != o.out ? out < o.out : host < o.host); } };
 
+// A step over several sessions (batched or mixed, see plan_step): segment i is len_i consecutive tokens of one session, the
+// columns of the step are the segments back to back.
+struct StepPlan {
+    std::vector<int2> segs;            // (session, len)
+    std::vector<int4> cols;            // column -> (session, position, T = n_past + len of its segment, 0)
+    std::vector<AttnBlock> blocks;     // head size 128: query blocks of the chunks on k_attn128_tiled
+    std::vector<int> clist;            // head size 128: the other columns (k_attn128<false>)
+    int t_rows = 0;                    // largest T among the tiled chunks
+    bool ones = true;                  // every segment is one token: the batched-step schedule (fused RoPE + attention)
+};
+
 }  // namespace b200
 
 using namespace b200;
@@ -52,7 +63,9 @@ struct b200_slice {
     std::vector<int> past;                 // n_past per session
     int * d_npast = nullptr;               // [n_sessions], device copy (graph replays read it)
     size_t sess_stride = 0;                // elements between two sessions' KV caches
-    int2 * d_cols = nullptr; const int2 * cols = nullptr;   // batched step: column -> (session, position)
+    // multi-session step: s->plan's tables on the device; cols != nullptr while such a step is being enqueued
+    int4 * d_cols = nullptr; const int4 * cols = nullptr; AttnBlock * d_blocks = nullptr; int * d_clist = nullptr;
+    StepPlan plan;
     std::vector<LayerW> layers;
     std::vector<void *> allocs;
     uint16_t * kc = nullptr, * vc = nullptr, * q16 = nullptr;
@@ -529,6 +542,18 @@ static int launch_persistent(b200_slice * s, const float * in, float * out) {
     return 0;
 }
 
+// query-tiled prompt attention over grid_y query blocks; ta.t_rows = the largest T the blocks see
+static int launch_attn_tiled(b200_slice * s, AttnTiledArgs ta, int grid_y) {
+    ta.t_pad = (ta.t_rows + 31) & ~31;
+    const size_t tsm = (size_t) ta.t_rows * kAttnRow + (size_t) kAttnQB * ta.t_pad * 6 + 4 * 8 * 128 * 4 + kAttnQB * 256 + 64;
+    static bool tattr[16] = {false};
+    if (!tattr[s->device & 15]) {
+        B200_CUDA(cudaFuncSetAttribute(k_attn128_tiled, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+        tattr[s->device & 15] = true;
+    }
+    return launch_simple(s, k_attn128_tiled, dim3(s->H, grid_y, 1), dim3(512, 1, 1), tsm, ta);
+}
+
 // ---------------------------------------------------------------- one forward over the slice
 // Enqueue every layer for N tokens at device-side position *d_npast (tensor_processor.cpp:537-766).
 static int enqueue_layers(b200_slice * s, const float * in, int N, float * out) {
@@ -587,13 +612,36 @@ static int enqueue_layers(b200_slice * s, const float * in, int N, float * out) 
             const bool preq = s->wtype != kWT_F16;
             const float dsc = wt_nibbles(s->wtype) ? 0.0625f : 1.0f;
             if (preq) { aa.aq_out = s->aq_att; aa.da_out = s->da_att; aa.out_nbq = s->nbqE; aa.out_dscale = dsc; aa.out_soff = s->soffE; }
-            if (s->cols) {
+            AttnTiledArgs ta{};
+            ta.q16 = s->q16; ta.kc = kc; ta.vc = vc; ta.n_past = d_npast; ta.E = E; ta.H = H; ta.N = N; ta.texp = s->texp; ta.out = s->att;
+            if (preq) { ta.aq_out = s->aq_att; ta.da_out = s->da_att; ta.out_nbq = s->nbqE; ta.out_dscale = dsc; ta.out_soff = s->soffE; }
+            ta.kq_scale = aa.kq_scale;
+            if (s->cols && s->plan.ones) {
                 // every column is an independent N = 1 step: the fused (RoPE + append) kernel, one cluster row per column
                 s->cur_class = 2;
                 for (int n0 = 0; n0 < N; n0 += kChunk) {
                     aa.n0 = n0;
                     const int cnt = N - n0 < kChunk ? N - n0 : kChunk;
                     if ((rc = launch_simple(s, k_attn128<true>, dim3(4 * H, cnt, 1), dim3(256, 1, 1), asm_bytes, aa))) return rc;
+                }
+            } else if (s->cols) {
+                // mixed step: every RoPE + KV append first (a chunk's queries read the rows the other columns of their segment
+                // append), then the tiled kernel over the query blocks of the chunks whose context fits the staged window, and
+                // the cluster kernel over every other column
+                s->cur_class = 1;
+                RopeArgs ra{s->qkv, E, H, D, N, d_npast, s->cs, s->q16, kc, vc, s->cols, s->sess_stride};
+                if ((rc = launch_simple(s, k_rope_append, dim3((E / 2 + 255) / 256, N, 1), dim3(256, 1, 1), 0, ra))) return rc;
+                s->cur_class = 2;
+                if (!s->plan.blocks.empty()) {
+                    ta.blocks = s->d_blocks; ta.sess_stride = s->sess_stride; ta.t_rows = s->plan.t_rows;
+                    if ((rc = launch_attn_tiled(s, ta, (int) s->plan.blocks.size()))) return rc;
+                }
+                aa.colmap = s->d_clist;
+                const int ncl = (int) s->plan.clist.size();
+                for (int n0 = 0; n0 < ncl; n0 += kChunk) {
+                    aa.n0 = n0;
+                    const int cnt = ncl - n0 < kChunk ? ncl - n0 : kChunk;
+                    if ((rc = launch_simple(s, k_attn128<false>, dim3(4 * H, cnt, 1), dim3(256, 1, 1), asm_plain, aa))) return rc;
                 }
             } else if (N == 1) {
                 s->cur_class = 2;
@@ -607,18 +655,8 @@ static int enqueue_layers(b200_slice * s, const float * in, int N, float * out) 
                 RopeArgs ra{s->qkv, E, H, D, N, d_npast, s->cs, s->q16, kc, vc, nullptr, 0};
                 if ((rc = launch_simple(s, k_rope_append, dim3((E / 2 + 255) / 256, N, 1), dim3(256, 1, 1), 0, ra))) return rc;
                 s->cur_class = 2;
-                const int Tn = s->past[s->cur] + N;
-                AttnTiledArgs ta{};
-                ta.q16 = s->q16; ta.kc = kc; ta.vc = vc; ta.n_past = d_npast; ta.E = E; ta.H = H; ta.N = N; ta.texp = s->texp; ta.out = s->att;
-                if (preq) { ta.aq_out = s->aq_att; ta.da_out = s->da_att; ta.out_nbq = s->nbqE; ta.out_dscale = dsc; ta.out_soff = s->soffE; }
-                ta.kq_scale = aa.kq_scale; ta.t_rows = Tn; ta.t_pad = (Tn + 31) & ~31;
-                const size_t tsm = (size_t) ta.t_rows * kAttnRow + (size_t) kAttnQB * ta.t_pad * 6 + 4 * 8 * 128 * 4 + kAttnQB * 256 + 64;
-                static bool tattr[16] = {false};
-                if (!tattr[s->device & 15]) {
-                    B200_CUDA(cudaFuncSetAttribute(k_attn128_tiled, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
-                    tattr[s->device & 15] = true;
-                }
-                if ((rc = launch_simple(s, k_attn128_tiled, dim3(H, (N + kAttnQB - 1) / kAttnQB, 1), dim3(512, 1, 1), tsm, ta))) return rc;
+                ta.t_rows = s->past[s->cur] + N;
+                if ((rc = launch_attn_tiled(s, ta, (N + kAttnQB - 1) / kAttnQB))) return rc;
             } else {
                 s->cur_class = 1;
                 RopeArgs ra{s->qkv, E, H, D, N, d_npast, s->cs, s->q16, kc, vc, nullptr, 0};
@@ -722,7 +760,7 @@ static int enqueue_layers(b200_slice * s, const float * in, int N, float * out) 
         cfg.attrs = at; cfg.numAttrs = s->use_pdl ? 1 : 0;
         s->cur_class = 6;
         prof_begin(s);
-        if (s->cols) B200_CUDA(cudaLaunchKernelEx(&cfg, k_advance_cols, s->d_npast, s->cols, N));
+        if (s->cols) B200_CUDA(cudaLaunchKernelEx(&cfg, k_advance_segs, s->d_npast, s->cols, N));
         else if (s->fold_send) B200_CUDA(cudaLaunchKernelEx(&cfg, k_advance_sent, s->d_npast + s->cur, N, (MailboxHdr *) s->mb_block));
         else         B200_CUDA(cudaLaunchKernelEx(&cfg, k_advance, s->d_npast + s->cur, N));
         prof_end(s);
@@ -811,44 +849,93 @@ static int forward_locked(b200_slice * s, const float * in, int N, float * out, 
     return 0;
 }
 
-// One token for each of B distinct sessions in a single pass: the weight matmuls see B columns (weights read once),
-// attention / RoPE / KV append run per column against that session's cache at that session's position.  Every column
-// is arithmetically the N = 1 step of its own sequence, so results are bit-identical to stepping the sessions one by one.
-static int batch_locked(b200_slice * s, const int * sessions, int B, const float * in, float * out, bool host) {
-    if (B <= 0 || B > s->n_sessions || B > s->n_ctx) return fail(B200_EINVAL, "batch of %d sequences with %d sessions", B, s->n_sessions);
-    std::vector<int2> cols(B);
+// A step over n_seg DISTINCT sessions in a single pass: segment i is n_tokens[i] consecutive tokens of sessions[i] (n_tokens
+// == nullptr: one token each, the batched step).  The weight matmuls see all columns at once (weights read once); RoPE, KV
+// append and attention run per column against that session's cache.  Column n of segment i carries T_i = n_past_i + len_i,
+// the row length the reference's V.p of that call splits into 32-slot body and double tail, so every segment's rows are
+// bit-identical to a forward of that session alone.  Checks every segment before anything is enqueued: a rejected step changes
+// nothing.  Fills s->plan; *rows = the step's column count.
+static int plan_step(b200_slice * s, const int * sessions, const int * n_tokens, int n_seg, int * rows) {
+    if (n_seg <= 0 || n_seg > s->n_sessions) return fail(B200_EINVAL, "step over %d sessions with %d sessions", n_seg, s->n_sessions);
     std::vector<char> seen(s->n_sessions, 0);
-    for (int b = 0; b < B; b++) {
-        const int k = sessions[b];
+    long long total = 0;
+    for (int i = 0; i < n_seg; i++) {
+        const int k = sessions[i], len = n_tokens ? n_tokens[i] : 1;
         if (k < 0 || k >= s->n_sessions) return fail(B200_EINVAL, "session %d outside [0, %d)", k, s->n_sessions);
-        if (seen[k]) return fail(B200_EINVAL, "session %d listed twice in one batched step", k);
+        if (seen[k]) return fail(B200_EINVAL, "session %d listed twice in one step", k);
+        if (len <= 0) return fail(B200_EINVAL, "segment %d of session %d has %d tokens", i, k, len);
         seen[k] = 1;
-        if (s->past[k] + 1 > s->n_ctx) return fail(B200_ECONTEXT, "context overflow: session %d n_past %d + 1 > n_ctx %d", k, s->past[k], s->n_ctx);
-        cols[b] = make_int2(k, s->past[k]);
+        total += len;
     }
+    if (total > s->n_ctx) return fail(B200_EINVAL, "step of %lld tokens exceeds n_ctx %d", total, s->n_ctx);
+    for (int i = 0; i < n_seg; i++) {
+        const int k = sessions[i], len = n_tokens ? n_tokens[i] : 1;
+        if (s->past[k] + len > s->n_ctx)
+            return fail(B200_ECONTEXT, "context overflow: session %d n_past %d + %d > n_ctx %d", k, s->past[k], len, s->n_ctx);
+    }
+    StepPlan & P = s->plan;
+    P.segs.clear(); P.cols.clear(); P.blocks.clear(); P.clist.clear(); P.t_rows = 0; P.ones = true;
+    for (int i = 0; i < n_seg; i++) {
+        const int k = sessions[i], len = n_tokens ? n_tokens[i] : 1, p0 = s->past[k], T = p0 + len, c0 = (int) P.cols.size();
+        P.segs.push_back(make_int2(k, len));
+        P.ones = P.ones && len == 1;
+        for (int j = 0; j < len; j++) P.cols.push_back(make_int4(k, p0 + j, T, 0));
+        // head size 128: the same choice a prompt chunk of this session alone gets (enqueue_layers, N > 1)
+        if (s->D == 128 && len > 1 && s->use_tiled_attn && T <= kAttnTMax) {
+            for (int j = 0; j < len; j += kAttnQB) P.blocks.push_back(AttnBlock{c0 + j, std::min(kAttnQB, len - j), k, p0 + j, T});
+            P.t_rows = std::max(P.t_rows, T);
+        } else {
+            for (int j = 0; j < len; j++) P.clist.push_back(c0 + j);
+        }
+    }
+    *rows = (int) total;
+    return 0;
+}
+
+// Copy s->plan's tables to the device and put the slice in multi-session mode (s->cols) for enqueue_layers.
+static int upload_plan(b200_slice * s) {
+    const StepPlan & P = s->plan;
+    // pageable sources: the driver stages them before returning, so the next plan may overwrite the vectors
+    B200_CUDA(cudaMemcpyAsync(s->d_cols, P.cols.data(), P.cols.size() * sizeof(int4), cudaMemcpyHostToDevice, s->stream));
+    if (!P.ones && !P.blocks.empty())
+        B200_CUDA(cudaMemcpyAsync(s->d_blocks, P.blocks.data(), P.blocks.size() * sizeof(AttnBlock), cudaMemcpyHostToDevice, s->stream));
+    if (!P.ones && !P.clist.empty())
+        B200_CUDA(cudaMemcpyAsync(s->d_clist, P.clist.data(), P.clist.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
+    s->cur = 0; s->cols = s->d_cols;
+    return 0;
+}
+
+static void commit_plan(b200_slice * s) { for (const int2 & g : s->plan.segs) s->past[g.x] += g.y; }
+
+// Enqueue the step s->plan describes (N columns) and advance its sessions.
+static int run_plan(b200_slice * s, int N, const float * in, float * out, bool host) {
+    int rc;
     B200_CUDA(cudaSetDevice(s->device));
     B200_CUDA(cudaEventRecord(s->ev0, s->stream));
-    // pageable source: the driver stages it before returning, so the vector may go out of scope
-    B200_CUDA(cudaMemcpyAsync(s->d_cols, cols.data(), (size_t) B * sizeof(int2), cudaMemcpyHostToDevice, s->stream));
-    s->cur = 0; s->cols = s->d_cols;
-    int rc;
+    if ((rc = upload_plan(s))) { s->cols = nullptr; return rc; }
     if (host) {
-        B200_CUDA(cudaMemcpyAsync(s->d_in, in, (size_t) B * s->E * 4, cudaMemcpyHostToDevice, s->stream));
-        rc = enqueue_layers(s, s->d_in, B, s->d_out);
+        B200_CUDA(cudaMemcpyAsync(s->d_in, in, (size_t) N * s->E * 4, cudaMemcpyHostToDevice, s->stream));
+        rc = enqueue_layers(s, s->d_in, N, s->d_out);
         s->cols = nullptr;
         if (rc) return rc;
         B200_CUDA(cudaEventRecord(s->ev1, s->stream));
-        B200_CUDA(cudaMemcpyAsync(out, s->d_out, (size_t) B * s->E * 4, cudaMemcpyDeviceToHost, s->stream));
+        B200_CUDA(cudaMemcpyAsync(out, s->d_out, (size_t) N * s->E * 4, cudaMemcpyDeviceToHost, s->stream));
         B200_CUDA(cudaStreamSynchronize(s->stream));
     } else {
-        rc = enqueue_layers(s, in, B, out);
+        rc = enqueue_layers(s, in, N, out);
         s->cols = nullptr;
         if (rc) return rc;
         B200_CUDA(cudaEventRecord(s->ev1, s->stream));
     }
     s->timed = true;
-    for (int b = 0; b < B; b++) s->past[sessions[b]] += 1;
+    commit_plan(s);
     return 0;
+}
+
+static int mixed_locked(b200_slice * s, const int * sessions, const int * n_tokens, int n_seg, const float * in, float * out, bool host) {
+    int N = 0;
+    const int rc = plan_step(s, sessions, n_tokens, n_seg, &N);
+    return rc ? rc : run_plan(s, N, in, out, host);
 }
 
 // ---------------------------------------------------------------- loader
@@ -1119,7 +1206,8 @@ static int load_locked(b200_slice * s, const char * path) {
     s->sess_stride = (size_t) s->L * nE;
     s->past.assign(s->n_sessions, 0);
     if ((rc = dev_alloc(s, &s->kc, s->n_sessions * s->sess_stride)) || (rc = dev_alloc(s, &s->vc, s->n_sessions * s->sess_stride)) ||
-        (rc = dev_alloc(s, &s->d_cols, (size_t) s->n_ctx)) ||
+        (rc = dev_alloc(s, &s->d_cols, (size_t) s->n_ctx)) || (rc = dev_alloc(s, &s->d_blocks, (size_t) s->n_ctx)) ||
+        (rc = dev_alloc(s, &s->d_clist, (size_t) s->n_ctx)) ||
         (rc = dev_alloc(s, &s->q16, nE)) || (rc = dev_alloc(s, &s->xa, nE)) || (rc = dev_alloc(s, &s->xb, nE)) ||
         (rc = dev_alloc(s, &s->qkv, 3 * nE)) || (rc = dev_alloc(s, &s->att, nE)) || (rc = dev_alloc(s, &s->ffin, nE)) ||
         (rc = dev_alloc(s, &s->gate, (size_t) s->n_ctx * FF)) || (rc = dev_alloc(s, &s->d_in, nE)) ||
@@ -1371,13 +1459,38 @@ int b200_session_forward_device(b200_slice_t * s, int session, const float * d_i
 int b200_batch_forward(b200_slice_t * s, const int * sessions, int n_seq, const float * in, float * out) {
     if (!s || !sessions || !in || !out) return fail(B200_EINVAL, "null argument");
     std::lock_guard<std::mutex> lk(s->mu);
-    return batch_locked(s, sessions, n_seq, in, out, true);
+    return mixed_locked(s, sessions, nullptr, n_seq, in, out, true);
 }
 
 int b200_batch_forward_device(b200_slice_t * s, const int * sessions, int n_seq, const float * d_in, float * d_out, int sync) {
     if (!s || !sessions || !d_in || !d_out) return fail(B200_EINVAL, "null argument");
     std::lock_guard<std::mutex> lk(s->mu);
-    int rc = batch_locked(s, sessions, n_seq, d_in, d_out, false);
+    int rc = mixed_locked(s, sessions, nullptr, n_seq, d_in, d_out, false);
+    if (rc) return rc;
+    if (sync) B200_CUDA(cudaStreamSynchronize(s->stream));
+    return 0;
+}
+
+// The mixed-step entry points are new: a caller without a device cannot have a handle, so a null handle reports why.
+static int null_handle() {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(B200_ENODEV, "no CUDA device visible: the slice forward has no CPU fallback");
+    return fail(B200_EINVAL, "null handle");
+}
+
+int b200_mixed_forward(b200_slice_t * s, const int * sessions, const int * n_tokens, int n_seg, const float * in, float * out) {
+    if (!s) return null_handle();
+    if (!sessions || !n_tokens || !in || !out) return fail(B200_EINVAL, "null argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    return mixed_locked(s, sessions, n_tokens, n_seg, in, out, true);
+}
+
+int b200_mixed_forward_device(b200_slice_t * s, const int * sessions, const int * n_tokens, int n_seg, const float * d_in, float * d_out,
+                              int sync) {
+    if (!s) return null_handle();
+    if (!sessions || !n_tokens || !d_in || !d_out) return fail(B200_EINVAL, "null argument");
+    std::lock_guard<std::mutex> lk(s->mu);
+    int rc = mixed_locked(s, sessions, n_tokens, n_seg, d_in, d_out, false);
     if (rc) return rc;
     if (sync) B200_CUDA(cudaStreamSynchronize(s->stream));
     return 0;
@@ -1638,7 +1751,7 @@ int b200_pipeline_init(b200_slice_t * s, int rank, int nranks, const void * id12
 // store into the next rank's mailbox + a flag, issued by k_peer_send right behind this slice's last matmul and picked
 // up by k_peer_recv in front of the next slice's first matmul.  For a single-token step the whole sequence
 // [recv ->] layers -> send [-> recv of the ring result] is ONE captured graph per rank: no host code between slices.
-static int pipeline_step_peer(b200_slice * s, const float * d_in, int n_rows, int ring, int session, const int * sessions) {
+static int pipeline_step_peer(b200_slice * s, const float * d_in, int n_rows, int ring, int session, bool multi) {
     const int r = s->pp_rank, W = s->pp_world;
     const size_t count = (size_t) n_rows * s->E;
     if (count > s->mb_slot_floats) return fail(B200_EINVAL, "hand-off of %zu floats exceeds the mailbox slot (%zu)", count, s->mb_slot_floats);
@@ -1649,13 +1762,13 @@ static int pipeline_step_peer(b200_slice * s, const float * d_in, int n_rows, in
     PeerRecvArgs rf = ra; rf.dst = s->d_final;
     PeerSendArgs sa{mine, (uint2 *)(s->mb_next + sizeof(MailboxHdr)), s->mb_slot_floats, s->d_out, (int) count};
     const int xfer_ctas = (int) std::min<size_t>(32, (count + 8191) / 8192);      // one CTA per 8 K elements, at most 32
-    if (!sessions) { s->cur = session; s->cols = nullptr; }
+    if (!multi) { s->cur = session; s->cols = nullptr; }
     // fold the send into the slice's last matmul for plain single-token steps of quantised, head-size-128 slices
-    const bool fold = s->use_fold && sends && !sessions && n_rows == 1 && s->D == 128 && s->wtype != kWT_F16 && s->use_ring && !s->use_nq &&
+    const bool fold = s->use_fold && sends && !multi && n_rows == 1 && s->D == 128 && s->wtype != kWT_F16 && s->use_ring && !s->use_nq &&
                       !persist_applicable(s, 1) && !s->skip_attention;
     const float * in = recv_in ? s->d_in : d_in;
     int rc = 0;
-    if (!sessions && persist_applicable(s, n_rows) && (rc = persist_prepare(s, in, s->d_out))) return rc;
+    if (!multi && persist_applicable(s, n_rows) && (rc = persist_prepare(s, in, s->d_out))) return rc;
     auto body = [&]() -> int {
         int e;
         s->cur_class = 6;
@@ -1670,15 +1783,12 @@ static int pipeline_step_peer(b200_slice * s, const float * d_in, int n_rows, in
         return 0;
     };
     B200_CUDA(cudaEventRecord(s->ev0, s->stream));
-    if (sessions) {
-        std::vector<int2> cols(n_rows);
-        for (int b = 0; b < n_rows; b++) cols[b] = make_int2(sessions[b], s->past[sessions[b]]);
-        B200_CUDA(cudaMemcpyAsync(s->d_cols, cols.data(), (size_t) n_rows * sizeof(int2), cudaMemcpyHostToDevice, s->stream));
-        s->cur = 0; s->cols = s->d_cols;
+    if (multi) {
+        if ((rc = upload_plan(s))) { s->cols = nullptr; return rc; }
         rc = body();
         s->cols = nullptr;
         if (rc) return rc;
-        for (int b = 0; b < n_rows; b++) s->past[sessions[b]] += 1;
+        commit_plan(s);
     } else if (n_rows == 1 && s->use_graph && !s->profiling) {
         GraphKey key{in, nullptr, (ring & 3) | (fold ? 4 : 0) | (session << 3)};
         auto it = s->pp_graphs.find(key);
@@ -1712,38 +1822,32 @@ static int pipeline_step_peer(b200_slice * s, const float * d_in, int n_rows, in
 }
 
 // recv <- rank-1, the slice's layers, send -> rank+1 (ring: the last rank hands its output back to rank 0).
-// sessions == nullptr: n_rows tokens of session `session`; else one token for each of the n_rows listed sessions.
-static int pipeline_step_locked(b200_slice * s, const float * d_in, int n_rows, int ring, int session, const int * sessions) {
+// sessions == nullptr: n_rows tokens of session `session`; else a step over the n_rows listed sessions, n_tokens[i] tokens of
+// sessions[i] (n_tokens == nullptr: one each), as b200_mixed_forward.
+static int pipeline_step_locked(b200_slice * s, const float * d_in, int n_rows, int ring, int session, const int * sessions,
+                                const int * n_tokens = nullptr) {
     NcclApi & n = nccl();
     B200_CUDA(cudaSetDevice(s->device));
-    if (n_rows <= 0 || n_rows > s->n_ctx) return fail(B200_EINVAL, "n_tokens %d outside [1, n_ctx]", n_rows);
-    const size_t count = (size_t) n_rows * s->E;
-    const int r = s->pp_rank, W = s->pp_world;
     int rc;
     // validate the step BEFORE anything is posted: a rejected step must not leave the peer's send unmatched
     if (sessions) {
-        if (n_rows > s->n_sessions) return fail(B200_EINVAL, "batch of %d sequences with %d sessions", n_rows, s->n_sessions);
-        std::vector<char> seen(s->n_sessions, 0);
-        for (int b = 0; b < n_rows; b++) {
-            const int k = sessions[b];
-            if (k < 0 || k >= s->n_sessions) return fail(B200_EINVAL, "session %d outside [0, %d)", k, s->n_sessions);
-            if (seen[k]) return fail(B200_EINVAL, "session %d listed twice in one batched step", k);
-            seen[k] = 1;
-            if (s->past[k] + 1 > s->n_ctx) return fail(B200_ECONTEXT, "context overflow: session %d n_past %d + 1 > n_ctx %d", k, s->past[k], s->n_ctx);
-        }
+        if ((rc = plan_step(s, sessions, n_tokens, n_rows, &n_rows))) return rc;
     } else {
+        if (n_rows <= 0 || n_rows > s->n_ctx) return fail(B200_EINVAL, "n_tokens %d outside [1, n_ctx]", n_rows);
         if (session < 0 || session >= s->n_sessions) return fail(B200_EINVAL, "session %d outside [0, %d)", session, s->n_sessions);
         if (s->past[session] + n_rows > s->n_ctx)
             return fail(B200_ECONTEXT, "context overflow: n_past %d + n_tokens %d > n_ctx %d", s->past[session], n_rows, s->n_ctx);
     }
+    const size_t count = (size_t) n_rows * s->E;
+    const int r = s->pp_rank, W = s->pp_world;
     if (r == 0 && !d_in) return fail(B200_EINVAL, "rank 0 needs an input buffer");
-    if (s->mb_on && W > 1) return pipeline_step_peer(s, d_in, n_rows, ring, session, sessions);
+    if (s->mb_on && W > 1) return pipeline_step_peer(s, d_in, n_rows, ring, session, sessions != nullptr);
     const float * in = d_in;
     if (r > 0) {
         if ((rc = n.Recv(s->d_in, count, kNcclFloat32, r - 1, s->nccl_comm, s->stream))) return nccl_fail("ncclRecv", rc);
         in = s->d_in;
     }
-    if (sessions) rc = batch_locked(s, sessions, n_rows, in, s->d_out, false);
+    if (sessions) rc = run_plan(s, n_rows, in, s->d_out, false);
     else          rc = forward_locked(s, in, n_rows, s->d_out, false, session);
     if (rc) return rc;
     if (r < W - 1) {
@@ -1776,6 +1880,14 @@ int b200_pipeline_step_batch(b200_slice_t * s, const int * sessions, int n_seq, 
     if (!sessions) return fail(B200_EINVAL, "null session list");
     std::lock_guard<std::mutex> lk(s->mu);
     return pipeline_step_locked(s, d_in, n_seq, ring, 0, sessions);
+}
+
+int b200_pipeline_step_mixed(b200_slice_t * s, const int * sessions, const int * n_tokens, int n_seg, const float * d_in, int ring) {
+    if (!s) return null_handle();
+    if (!s->nccl_comm) return fail(B200_EINVAL, "pipeline not initialised");
+    if (!sessions || !n_tokens) return fail(B200_EINVAL, "null session list");
+    std::lock_guard<std::mutex> lk(s->mu);
+    return pipeline_step_locked(s, d_in, n_seg, ring, 0, sessions, n_tokens);
 }
 
 /* ---- peer-memory hand-off: mailboxes mapped across processes with cudaIpc --------------------------------------- */

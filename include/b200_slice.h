@@ -101,12 +101,23 @@ int b200_session_forward_device(b200_slice_t * s, int session, const float * d_i
 int b200_batch_forward(b200_slice_t * s, const int * sessions, int n_seq, const float * in, float * out);      /* host buffers */
 int b200_batch_forward_device(b200_slice_t * s, const int * sessions, int n_seq, const float * d_in, float * d_out, int sync);
 
+/* Mixed step (continuous batching): for each of n_seg DISTINCT sessions, n_tokens[i] >= 1 consecutive tokens of that session,
+ * all in ONE pass -- a new session's prompt chunk rides in the same weight pass as the other sessions' decode tokens.  in / out
+ * are [sum n_tokens][n_embd], the segments back to back in the listed order.  Segment i's rows are bit-identical to
+ * b200_session_forward(sessions[i], <its rows>, n_tokens[i]) on the state before the call, whatever the other segments are;
+ * b200_batch_forward is the case n_tokens[i] = 1.  Always exact mode: the fast-prefill switch is ignored.
+ * A session listed twice, n_tokens[i] <= 0, a session out of range, or sum n_tokens > n_ctx -> B200_EINVAL; a session with
+ * n_past + n_tokens[i] > n_ctx -> B200_ECONTEXT.  A rejected step advances no session.  No device: B200_ENODEV. */
+int b200_mixed_forward(b200_slice_t * s, const int * sessions, const int * n_tokens, int n_seg, const float * in, float * out);   /* host buffers */
+int b200_mixed_forward_device(b200_slice_t * s, const int * sessions, const int * n_tokens, int n_seg,
+                              const float * d_in, float * d_out, int sync);
+
 /* Fast mode for prefill calls (n_tokens >= min_tokens): the Q4_0 / Q8_0 weight matmuls run on the tcgen05 tensor cores with
  * the dequantisation fused in (csrc/fastgemm2.cuh; Q4_1 and F16 slices ignore the switch and stay exact).  NOT bit-exact: operands are rounded to fp16 after the reference's
  * Q8_0 activation quantisation; deviation from exact mode is bounded in tests/test_gpu_fast_prefill.py and, one matmul at a
  * time, in tests/test_gpu_fast_matmul.py.  The fp16 operands limit the un-normalised inputs of wo and w2 to |x| <= 65504;
  * beyond that fast mode overflows where exact mode stays finite.  Off by default (or B200_FAST_PREFILL=1).  Single-token
- * steps and batched steps (b200_batch_forward*) always run in exact mode, whatever min_tokens is: only a multi-token call of
+ * steps, batched steps (b200_batch_forward*) and mixed steps (b200_mixed_forward*) always run in exact mode, whatever min_tokens is: only a multi-token call of
  * one sequence takes the fast path. */
 int b200_slice_set_fast_prefill(b200_slice_t * s, int on, int min_tokens);
 
@@ -184,6 +195,9 @@ int b200_pipeline_step(b200_slice_t * s, const float * d_in, int n_tokens, int r
  * between the slices).  Every rank passes the same session list. */
 int b200_pipeline_step_session(b200_slice_t * s, int session, const float * d_in, int n_tokens, int ring);
 int b200_pipeline_step_batch(b200_slice_t * s, const int * sessions, int n_seq, const float * d_in, int ring);
+/* The same hand-off for a mixed step ([sum n_tokens][n_embd] moves between the slices; see b200_mixed_forward).  Every rank
+ * passes the same segment list; a rejected list is rejected on every rank before anything is sent or received. */
+int b200_pipeline_step_mixed(b200_slice_t * s, const int * sessions, const int * n_tokens, int n_seg, const float * d_in, int ring);
 /* Peer-memory hand-off (the B200-native hop): every rank owns a MAILBOX in its HBM (sequence flags + two inbox slots of
  * [n_ctx][n_embd] f32) that its ring neighbours map over NVLink with cudaIpc.  After b200_pipeline_init, each rank
  * exports its 64-byte handle, the host gathers all of them (torch.distributed all_gather, a file, ...) and every rank
